@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the openrec.tf2 training step on B200: BPR (headline), UCML, DLRM; roofline + CPU baseline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload bpr|ucml|dlrm] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload bpr|ucml|dlrm] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workloads (BASELINE.json configs): bpr = configs[1] (N = 1) / configs[4] shape (N > 1), ucml = configs[2],
@@ -49,6 +49,10 @@ METRICS = {"bpr": ("bpr_triplets_per_sec", "triplets/s"), "ucml": ("ucml_triplet
 DLRM_T, DLRM_VOCAB, DLRM_B, DLRM_DENSE = 26, 1_000_000, 32_768, 13
 DLRM_BOT, DLRM_TOP = [512, 256, D], [1024, 1024, 512, 256, 1]
 DLRM_LR = 0.01
+# --dump-outputs: rows sampled from each 1M-row table, so that the three workloads together stay under DUMP_LIMIT
+# (BPR and UCML 2 MB per table, DLRM 26 x 0.5 MB of tables + 9 MB of MLP weights)
+DUMP_ROWS, DLRM_DUMP_ROWS = 4096, 1024
+DUMP_LIMIT = 64 << 20
 
 
 def dlrm_layers():
@@ -339,6 +343,24 @@ def _timed(fn_step, K, barrier, torch, clocks):
     return e0.elapsed_time(e1) * 1e-3
 
 
+def _sample_rows(t, n):
+    """n rows of a device tensor, picked by a fixed seed and kept in row order (all rows if it has no more), as float32."""
+    import torch
+    if t.shape[0] <= n:
+        return t.float().cpu().numpy()
+    idx = np.sort(np.random.default_rng(0).choice(t.shape[0], n, replace=False))
+    return t.index_select(0, torch.from_numpy(idx).to(t.device)).float().cpu().numpy()
+
+
+def write_dumps(out_dir, arrays):
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes, more than {DUMP_LIMIT}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def bench_pairwise(wl, args, eng, dev, barrier, clocks, with_extra=True):
     import torch
     from openrec_b200 import native as N
@@ -370,6 +392,10 @@ def bench_pairwise(wl, args, eng, dev, barrier, clocks, with_extra=True):
     for i in range(W):
         step(i - W)
     seconds = _timed(step, K, barrier, torch, clocks)
+    dump = {}
+    if args.dump_outputs:      # the last timed step's results, before the loops below train the same tables further
+        dump = {f"{wl}_loss_l2": out4[:2].cpu().numpy(), f"{wl}_user_rows": _sample_rows(tu, DUMP_ROWS),
+                f"{wl}_item_rows": _sample_rows(ti, DUMP_ROWS), f"{wl}_item_bias_rows": _sample_rows(tb, DUMP_ROWS)}
     loss_check = out4.cpu().numpy().tolist()
     # ---- roofline: the same loop, instrumented (events around the phases of every 8th step), >= 64 samples
     n_inst = 8 * 64 + 8
@@ -471,7 +497,7 @@ def bench_pairwise(wl, args, eng, dev, barrier, clocks, with_extra=True):
             "h2d": 3 * 4 * B, "d2h": 16,
             "e2e_api": f"openrec.tf2.recommenders.{'BPR' if wl == 'bpr' else 'UCML'} + tf.GradientTape + "
                        "tf.keras.optimizers.Adagrad (shim); pinned host ids in, loss read to host each step",
-            "extra": extra}
+            "extra": extra, "dump": dump}
 
 
 def bench_dlrm(args, eng, dev, barrier, clocks):
@@ -512,6 +538,11 @@ def bench_dlrm(args, eng, dev, barrier, clocks):
         step(i)
     seconds = _timed(step, K, barrier, torch, clocks)
     loss_value = float(state["prev"])
+    dump = {}
+    if args.dump_outputs:      # the last timed step's results, before the loops below train the same model further
+        dump["dlrm_loss"] = np.array([loss_value], dtype=np.float32)
+        for k, v in enumerate(model.trainable_variables):     # 26 embedding tables, then the MLP kernels and biases
+            dump[f"dlrm_var{k:02d}"] = _sample_rows(v.t, DLRM_DUMP_ROWS)
     # ---- roofline: the Dense-layer GEMMs (dominant kernels), timed with events around every GEMM call of a few steps
     prof = mlp_ops.GemmProfile()
     t0 = time.time()
@@ -551,7 +582,7 @@ def bench_dlrm(args, eng, dev, barrier, clocks):
             "h2d": DLRM_B * (DLRM_DENSE * 4 + DLRM_T * 4 + 4), "d2h": 4,
             "e2e_api": "openrec.tf2.recommenders.DLRM + tf.GradientTape + tf.keras.optimizers.Adagrad (shim); pinned host "
                        "dense / sparse / label in, loss read to host each step",
-            "extra": {"last_loss_value_path": loss_value, "last_loss_e2e": state["last"]}}
+            "extra": {"last_loss_value_path": loss_value, "last_loss_e2e": state["last"]}, "dump": dump}
 
 
 def make_line(wl, args, world, result, clocks_report, cpu=None):
@@ -634,6 +665,7 @@ def run_b200(args, rank, world, local_rank):
         return {"value": v, "unit": METRICS[w][1], **info}
 
     line = make_line(wl, args, 1, result, clocks_main, cpu_of(wl, cpu_budget))
+    dumps = dict(result["dump"])
     if wl == "bpr" and not args.no_secondary:
         line["secondary"] = []
         for w in ("ucml", "dlrm"):
@@ -642,9 +674,12 @@ def run_b200(args, rank, world, local_rank):
             try:
                 r = run[w]()
                 line["secondary"].append(make_line(w, args, 1, r, clocks.report(), cpu_of(w, cpu_budget / 2)))
+                dumps.update(r["dump"])
             except Exception as e:                                 # a secondary workload must never cost the headline line
                 line["secondary"].append({"metric": METRICS[w][0], "error": f"{type(e).__name__}: {e}"})
     clocks.report(final=True)
+    if args.dump_outputs:
+        write_dumps(args.dump_outputs, dumps)
     print(json.dumps(line), flush=True)
 
 
@@ -660,7 +695,13 @@ def main():
     ap.add_argument("--check", action="store_true",
                     help="--gpus N > 1: after the timed loops run ONE more step on a fresh batch and verify it on rank 0 against "
                          "the oracle over the rows the global batch touches (tests/shard_check.py); the verdict goes to extra.check")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="--gpus 1: write what the last timed step of each workload run computed to DIR/<name>.npy "
+                         "(float32): the loss, and the trained tables and weights, each table a fixed sample of "
+                         f"{DUMP_ROWS} (DLRM: {DLRM_DUMP_ROWS}) rows; the inputs depend only on the arguments")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.gpus != 1):
+        ap.error("--dump-outputs needs --impl b200 and --gpus 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -7,8 +7,13 @@ import subprocess
 import time
 
 import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+# staged by __graft_entry__.build() (oracle/build_ref.py) where the original checkout was readable
+REF_EXAMPLES = os.path.join(ROOT, "oracle", "_ref", "tf2_examples")
+needs_ref_examples = pytest.mark.skipif(not os.path.exists(os.path.join(REF_EXAMPLES, "bpr_citeulike.py")),
+                                        reason="original tf2_examples not staged under oracle/_ref/ by build()")
 
 RUNNER = r"""
 import sys, runpy

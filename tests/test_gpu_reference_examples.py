@@ -1,34 +1,29 @@
 """GPU: the reference's tf2_examples/bpr_citeulike.py and dlrm_criteo.py run UNMODIFIED against liborx.so -- the real
 kernels behind the reference's own class surface and step protocol (north_star: "tf2_examples/*.py run unmodified").
-The scripts are not part of this repo: tools/stage_reference_examples.py (run by __graft_entry__.build() in the build
-container) copies them into the git-ignored tests/_ref_examples/, which travels with the gpurun snapshot."""
-import os
+The scripts are not part of this repo: build() stages them into the git-ignored oracle/_ref/ (oracle/build_ref.py)
+where the original checkout is readable, and these tests skip where it staged nothing."""
 import subprocess
 import sys
 
 import pytest
 
-from _examples_common import check_bpr_line, check_dlrm_line, make_citeulike, make_criteo, run_until, runner_code
+from _examples_common import (REF_EXAMPLES, check_bpr_line, check_dlrm_line, make_citeulike, make_criteo,
+                              needs_ref_examples, run_until, runner_code)
 
-pytestmark = pytest.mark.gpu
-STAGED = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref_examples")
-needs_staged = pytest.mark.skipif(not os.path.exists(os.path.join(STAGED, "bpr_citeulike.py")),
-                                  reason="reference examples not staged (python tools/stage_reference_examples.py)")
+pytestmark = [pytest.mark.gpu, needs_ref_examples]
 
 
-@needs_staged
 def test_bpr_citeulike_runs_unmodified_on_gpu(tmp_path):
     work = make_citeulike(tmp_path)
-    out, ok = run_until([sys.executable, "-c", runner_code(STAGED, "bpr_citeulike.py", False)], str(work),
+    out, ok = run_until([sys.executable, "-c", runner_code(REF_EXAMPLES, "bpr_citeulike.py", False)], str(work),
                         [b"Iter: 0, Loss:", b"3 iter training."], 600)
     assert ok, out[-3000:]
     check_bpr_line(out)
 
 
-@needs_staged
 def test_dlrm_criteo_runs_unmodified_on_gpu(tmp_path):
     work = make_criteo(tmp_path)
-    r = subprocess.run([sys.executable, "-c", runner_code(STAGED, "dlrm_criteo.py", False)], cwd=str(work),
+    r = subprocess.run([sys.executable, "-c", runner_code(REF_EXAMPLES, "dlrm_criteo.py", False)], cwd=str(work),
                        capture_output=True, text=True, timeout=900)
     out = (r.stdout + r.stderr).replace("\r", "\n")
     assert r.returncode == 0, out[-3000:]

@@ -1,7 +1,8 @@
 """Dense-layer GEMM alone at the DLRM shapes (forward, dgrad, wgrad): CUDA-event time and fp32-equivalent TFLOP/s;
 also the ncu target for the tcgen05 kernel.   python tools/gemm_probe.py [reps]"""
+import os
 import sys
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from openrec_b200 import native as N
 eng = N.engine()
